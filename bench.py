@@ -1,13 +1,18 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the Show-o hot path on B200 (contract: see the task brief / DESIGN.md section 6).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...          (N > 1: one rank per GPU, NCCL)
 
 A "step" = one batch of the configs[1] workload of BASELINE.json on every rank: showo_demo.yaml t2i 256x256,
 18 denoise steps, CFG 5, batch 8 per GPU (weak scaling) -> t2i_generate + MAGVIT decode_code + uint8 conversion
 (SURVEY.md section 8d, config 2), then (N > 1) an NCCL all-gather of the uint8 images.
 Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR: after the timed steps, rank 0 saves what the last headline step returned to it as float32
+DIR/codes.npy ([8, 256] image-token ids from t2i_generate) and DIR/images.npy ([8, 256, 256, 3] uint8 pixel values),
+6.3 MB in all.  Weights, prompts and torch's RNG are seeded, so the same arguments give the same inputs on every run
+and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -191,6 +196,7 @@ def run_ours(args):
     torch.cuda.set_device(dev)
     P.init("nccl", dev)
     lib = _lib.require_gpu()
+    torch.manual_seed(0)          # t2i_generate draws its sampler seed from torch's RNG: identical runs for identical arguments
 
     model = showo_b200.Showo(False, V, 50295, materialize=False)
     model._make_engine(dev)
@@ -238,36 +244,42 @@ def run_ours(args):
             t4 = time.perf_counter()                           # host-side split of the e2e step (reported under e2e.host_phases_ms)
             phase_s["mask"] += t1 - t0; phase_s["generate_call"] += t2 - t1; phase_s["decode_call"] += t3 - t2; phase_s["tail_sync"] += t4 - t3
             e2e_step_ms.append(round(1e3 * (t4 - t0), 1))
-        return imgs
+        return codes, imgs
 
     def timed(e2e: bool, steps: int):
+        """device time of `steps` steps, and what the last one returned"""
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            one_step(e2e)
+            last = one_step(e2e)
         e1.record()
         torch.cuda.synchronize()
         ms = P.max_over_ranks(e0.elapsed_time(e1), dev)       # the slowest rank's device time
         if world > 1:
             dist.barrier()
-        return ms
+        return ms, last
 
     for _ in range(max(args.warmup, 3)):      # both call shapes warm up (first-use allocations, pinned-copy set-up, mempool creation)
         one_step(False)
         one_step(True)
     sampler = ClockSampler(local)
     sampler.start()
-    ms_dev = timed(False, args.steps)
+    ms_dev, (codes, imgs) = timed(False, args.steps)
     launches = model.kernel_launches() + vq.kernel_launches()
     for k in phase_s:
         phase_s[k] = 0.0
-    ms_e2e = timed(True, args.steps)
+    ms_e2e, _ = timed(True, args.steps)
     host_phases = {k: round(1e3 * v / args.steps, 2) for k, v in phase_s.items()}
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in (("codes", codes), ("images", imgs)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.float().cpu().numpy())
 
     # ---- secondaries run on EVERY rank (weak scaling like the headline) and are aggregated below
     if os.environ.get("SHOWO_BENCH_HEADLINE_ONLY"):           # A/B runs while tuning: the headline line only
@@ -744,7 +756,12 @@ if __name__ == "__main__":
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="save the last timed step's outputs as DIR/<name>.npy (float32)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if a.impl == "reference":
         run_reference(a)
     else:

@@ -21,6 +21,26 @@ def load(name):
     return np.load(os.path.join(HERE, name))
 
 
+def record_observed(name, key, value):
+    """Adds `key: value` to the JSON file `name` in $SHOWO_OBSERVED_DIR (nothing is written when it is unset).  The variant
+    tests run the parity tests in parallel processes that record into the same file, so each update holds an exclusive
+    lock on it from the read to the end of the write."""
+    import fcntl
+    import json
+    out = os.environ.get("SHOWO_OBSERVED_DIR")
+    if not out:
+        return
+    os.makedirs(out, exist_ok=True)
+    with open(os.path.join(out, name), "a+") as f:
+        fcntl.flock(f, fcntl.LOCK_EX)
+        f.seek(0)
+        text = f.read()
+        d = json.loads(text) if text else {}
+        d[key] = value
+        f.truncate(0)
+        json.dump(d, f, indent=1)
+
+
 def unpack_mask(z, key):
     shape = tuple(int(v) for v in z[key + "_shape"])
     n = int(np.prod(shape))

@@ -1,109 +1,114 @@
-"""Live pin of the oracle against the UNMODIFIED reference Python (only where /root/reference exists, i.e. the build
-container; the GPU box runs the committed golden vectors in test_oracle_golden.py instead)."""
+"""Pin of the oracle against the UNMODIFIED reference Python on the same seeded inputs: what the reference computed is stored in
+tests/golden/oracle_vs_reference.npz (tests/golden/make_golden_vs_reference.py ran it), so the comparison needs no reference
+checkout.  Large outputs are kept as a full-coverage digest (per-position argmax / logsumexp, per-row means) plus a fixed sample."""
+import numpy as np
 import pytest
 import torch
 
-import ref_loader as R
+import fixtures as FX
+import make_golden_vs_reference as G
 from oracle import magvit_oracle as MO
 from oracle import showo_oracle as O
 
-pytestmark = pytest.mark.skipif(not R.available(), reason="/root/reference not present on this box")
 VOC = O.ShowoVocab()
+
+
+@pytest.fixture(scope="module")
+def z():
+    return FX.load("oracle_vs_reference.npz")
 
 
 @pytest.fixture(scope="module")
 def tiny():
     dims = O.PhiDims(hidden=256, n_layers=2, n_heads=4, ffn=1024)
-    W = O.make_showo_weights(dims, seed=3)
-    model, mods = R.build_showo(dims, W)
-    return dims, W, model, mods
+    return dims, O.make_showo_weights(dims, seed=3)
 
 
-def test_state_dict_keys_match_reference(tiny):
-    dims, W, model, mods = tiny
-    ref_keys = {k for k in model.state_dict().keys() if "rotary_emb" not in k}
-    assert ref_keys == set(W.keys())
+def _require_reference_noise(z):
+    """the sampled paths replay torch's CPU noise streams: only comparable where they match the ones the reference drew"""
+    if not np.array_equal(G.noise_probe(), z["noise_probe"]):
+        pytest.skip("torch CPU exponential_ stream differs on this host; the sampled replay needs identical noise")
+
+
+def _mask(z, key):
+    allowed = FX.unpack_mask(z, key)
+    return torch.zeros(allowed.shape).masked_fill_(~allowed, float(z[key + "_neg"][0]))
+
+
+def test_state_dict_keys_match_reference(tiny, z):
+    dims, W = tiny
+    ref = {str(k): tuple(int(s) for s in str(v).split("x")) for k, v in zip(z["state_names"], z["state_shapes"])}
+    assert set(ref) == set(W.keys())
     import showo_b200
     ours = showo_b200.Showo(False, dims.vocab_size, VOC.llm_vocab_size, phi_dims=dict(hidden=256, n_layers=2, n_heads=4, ffn=1024))
-    assert set(ours.state_dict().keys()) == ref_keys
+    assert set(ours.state_dict().keys()) == set(ref)
     for k, v in ours.state_dict().items():
-        assert v.shape == model.state_dict()[k].shape, k
+        assert tuple(v.shape) == ref[k], k
 
 
-def test_masks_equal_reference(tiny):
-    _, _, _, mods = tiny
-    cond, uncond = O.make_t2i_prompts(3, VOC, seed=5)
-    ids = torch.cat([cond, uncond])
-    ref = mods.prompting.create_attention_mask_predict_next(ids, pad_id=O.PAD, soi_id=O.SOI, eoi_id=O.EOI, rm_pad_in_image=True)
-    assert torch.equal(ref, O.create_attention_mask_predict_next(ids))
-    ref2 = mods.prompting.create_attention_mask_predict_next(ids, pad_id=O.PAD, soi_id=O.SOI, eoi_id=O.EOI, rm_pad_in_image=False)
-    assert torch.equal(ref2, O.create_attention_mask_predict_next(ids, rm_pad_in_image=False))
-    codes = torch.randint(0, 8192, (2, 256))
-    mm = O.make_mmu_prompts(2, VOC, codes, q_len=9)
-    assert torch.equal(mods.prompting.create_attention_mask_for_mmu(mm, eoi_id=O.EOI), O.create_attention_mask_for_mmu(mm))
+def test_masks_equal_reference(z):
+    ids, mm = G.mask_case_rows()
+    assert torch.equal(_mask(z, "mask_t2i"), O.create_attention_mask_predict_next(ids))
+    assert torch.equal(_mask(z, "mask_t2i_keep_pad"), O.create_attention_mask_predict_next(ids, rm_pad_in_image=False))
+    assert torch.equal(_mask(z, "mask_mmu"), O.create_attention_mask_for_mmu(mm))
 
 
-def test_logits_and_t2i_generate_equal_reference(tiny):
-    dims, W, model, mods = tiny
+def test_logits_and_t2i_generate_equal_reference(tiny, z):
+    dims, W = tiny
     cond, uncond = O.make_t2i_prompts(2, VOC, seed=5)
     mask = O.create_attention_mask_predict_next(torch.cat([cond, uncond]))
     with torch.no_grad():
-        lr = model(torch.cat([cond, uncond]), attention_mask=mask)
         lo = O.showo_logits(W, dims, input_ids=torch.cat([cond, uncond]), add_mask=mask)
-    assert (lr - lo).abs().max().item() < 1e-5
-    for w, T in ((5.0, 4), (0.0, 3)):
-        g1, g2 = torch.Generator().manual_seed(11), torch.Generator().manual_seed(11)
-        c1, c2 = cond.clone(), cond.clone()
+    got = G.logits_summary(lo)
+    assert np.abs(got["sample"] - z["logits_sample"]).max() < 1e-5
+    assert np.abs(got["lse"] - z["logits_lse"]).max() < 1e-5
+    # the reference's argmax is (within the same bound) a maximum of ours: robust to exact ties
+    at_ref = lo.gather(-1, torch.from_numpy(z["logits_argmax"]).long()[..., None])[..., 0]
+    assert (lo.max(-1).values - at_ref).max().item() < 1e-5
+    _require_reference_noise(z)
+    for i, (w, T) in enumerate(G.T2I_CASES):
+        c2 = cond.clone()
         with torch.no_grad():
-            r = model.t2i_generate(input_ids=c1, uncond_input_ids=uncond.clone(), attention_mask=mask if w > 0 else mask[:2],
-                                   guidance_scale=w, timesteps=T, generator=g1, config=R.t2i_config(VOC))
             o = O.t2i_generate(W, dims, VOC, c2, uncond.clone(), mask if w > 0 else mask[:2], guidance_scale=w, timesteps=T,
-                               generator=g2)
-        assert torch.equal(r, o) and torch.equal(c1, c2)
+                               generator=torch.Generator().manual_seed(11))
+        assert np.array_equal(o.numpy(), z[f"t2i_ids_{i}"]) and np.array_equal(c2.numpy(), z[f"t2i_final_input_ids_{i}"])
 
 
-def test_mmu_generate_equals_reference(tiny):
-    dims, W, model, mods = tiny
-    codes = torch.randint(0, 8192, (1, 256), generator=torch.Generator().manual_seed(2))
-    mm = O.make_mmu_prompts(1, VOC, codes, q_len=7)
-    mk = O.create_attention_mask_for_mmu(mm)
+def test_mmu_generate_equals_reference(tiny, z):
+    dims, W = tiny
+    mm, mk = G.mmu_case_rows()
     with torch.no_grad():
-        r = model.mmu_generate(mm, attention_mask=mk, max_new_tokens=5, top_k=1)
         o = O.mmu_generate(W, dims, mm, mk, max_new_tokens=5, top_k=1)
-    assert torch.equal(torch.stack(r), torch.stack(o))
+    assert np.array_equal(torch.stack(o).numpy(), z["mmu_greedy"])
     # sampled decode (modeling_showo.py:219-228): temperature, top-k filter, softmax, torch.multinomial(p, 1) -- whose
     # single-sample path is the exponential race the oracle (and the CUDA kernel) restate; both draw from the global RNG
-    for top_k, temp in ((None, 0.8), (5, 1.3), (1, 0.5)):
-        torch.manual_seed(17)
-        with torch.no_grad():
-            r = model.mmu_generate(mm, attention_mask=mk, max_new_tokens=4, temperature=temp, top_k=top_k)
+    _require_reference_noise(z)
+    for i, (top_k, temp) in enumerate(G.MMU_SAMPLED_CASES):
         torch.manual_seed(17)
         with torch.no_grad():
             o = O.mmu_generate(W, dims, mm, mk, max_new_tokens=4, temperature=temp, top_k=top_k)
-        assert torch.equal(torch.stack(r), torch.stack(o)), (top_k, temp)
+        assert np.array_equal(torch.stack(o).numpy(), z[f"mmu_sampled_{i}"]), (top_k, temp)
 
 
-def test_magvit_equals_reference():
+def test_magvit_equals_reference(z):
     W = MO.make_magvit_weights(1)
-    vq, _ = R.build_magvit(W)
-    assert set(k for k in vq.state_dict() if not k.startswith("quantize.")) == set(W.keys())
-    x = torch.rand(1, 3, 256, 256, generator=torch.Generator().manual_seed(0)) * 2 - 1
-    ids = torch.randint(0, 8192, (1, 256), generator=torch.Generator().manual_seed(1))
+    assert set(str(k) for k in z["magvit_state_names"]) == set(W.keys())
+    x, ids = G.magvit_case_inputs()
     with torch.no_grad():
-        assert torch.equal(vq.get_code(x), MO.get_code(x, W))
-        assert (vq.decode_code(ids) - MO.decode_code(ids, W)).abs().max().item() < 1e-5
+        assert np.array_equal(MO.get_code(x, W).numpy(), z["magvit_codes"])
+        got = G.pixels_summary(MO.decode_code(ids, W))
+    assert np.abs(got["sample"] - z["magvit_decode_sample"]).max() < 1e-5
+    assert np.abs(got["row_mean"] - z["magvit_decode_row_mean"]).max() < 1e-5
 
 
-def test_mask_schedules_equal_reference(tiny):
+def test_mask_schedules_equal_reference(z):
     """get_mask_chedule (sic) and every schedule it hands out, bit for bit on the fp32 grid the sampler evaluates them on
     (models/sampling.py:39-78)."""
     import showo_b200
-    _, _, _, mods = tiny
-    ts = [torch.tensor(float(i) / 18) for i in range(19)] + [torch.rand(7, generator=torch.Generator().manual_seed(1))]
-    for method, kw in (("cosine", {}), ("linear", {}), ("pow2", {}), ("pow0.5", {}), ("pow3", {}), ("sigmoid", {}),
-                       ("sigmoid", dict(start=-2, end=4, tau=0.7))):
-        ref, ours = mods.sampling.get_mask_chedule(method, **kw), showo_b200.get_mask_chedule(method, **kw)
-        for t in ts:
-            assert torch.equal(ref(t), ours(t)), (method, t)
+    for i, (method, kw) in enumerate(G.SCHEDULES):
+        ours = showo_b200.get_mask_chedule(method, **kw)
+        vals = [ours(t) for t in G.schedule_points()]
+        assert all(v.dtype == torch.float32 for v in vals), method
+        assert np.array_equal(torch.cat([v.reshape(-1) for v in vals]).numpy(), z[f"schedule_{i}"]), (method, kw)
     with pytest.raises(ValueError):
         showo_b200.get_mask_chedule("nope")

@@ -1,21 +1,19 @@
-"""Static drop-in check (build container only: needs /root/reference): every call the reference's scripts make on the objects this repo
-replaces -- `model` (Showo), `vq_model` (MAGVITv2), `get_mask_chedule`, `mask_or_random_replace_tokens`, `uni_prompting` for the t2i rows
--- is parsed out of inference_t2i.py / inference_mmu.py / training/train.py and bound against the drop-in's signatures: the method has
-to exist and accept the positional count and every keyword the script passes (or swallow it through **kwargs like the reference does).
-The scripts cannot be executed here (no GPU) nor on the GPU box (no reference tree), so this is the strongest offline statement of
-"runs unchanged" besides the GPU tests that drive the same methods with the scripts' argument shapes."""
-import ast
+"""Static drop-in check: every call the reference's scripts make on the objects this repo replaces -- `model` (Showo), `vq_model`
+(MAGVITv2), `get_mask_chedule`, `mask_or_random_replace_tokens`, `uni_prompting` for the t2i rows -- was parsed out of inference_t2i.py /
+inference_mmu.py / training/train.py / training/train_w_clip_vit.py into tests/golden/reference_calls.json
+(tests/golden/make_golden_vs_reference.py) and is bound here against the drop-in's signatures: the method has to exist and accept the
+positional count and every keyword the script passes (or swallow it through **kwargs like the reference does).  Besides the GPU tests
+that drive the same methods with the scripts' argument shapes, this is the strongest offline statement of "runs unchanged"."""
 import inspect
+import json
 import os
 
 import pytest
 import torch
 
+import fixtures as FX
 import showo_b200
 from showo_b200 import train_inputs
-
-REF = os.environ.get("SHOWO_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")), reason="reference tree not present")
 
 # instances, not classes: mm_projector only exists on a w_clip_vit model (like in the reference)
 TARGETS = {"model": showo_b200.Showo(True, 58498, 50295, phi_dims=dict(hidden=128, n_layers=1, n_heads=2, ffn=256)),
@@ -30,20 +28,11 @@ SKIP_METHODS = {"to", "eval", "train", "requires_grad_", "parameters", "named_pa
                 "module", "get", "resize_token_embeddings"}
 
 
-def _calls(path):
-    tree = ast.parse(open(path).read())
-    out = []
-    for node in ast.walk(tree):
-        if not isinstance(node, ast.Call):
-            continue
-        f = node.func
-        if isinstance(f, ast.Attribute) and isinstance(f.value, ast.Name) and f.value.id in TARGETS:
-            out.append((f.value.id, f.attr, len(node.args), [k.arg for k in node.keywords if k.arg], node.lineno))
-        elif isinstance(f, ast.Name) and f.id in TARGETS:             # model(input_ids, ...)
-            out.append((f.id, "forward", len(node.args), [k.arg for k in node.keywords if k.arg], node.lineno))
-        elif isinstance(f, ast.Name) and f.id in FUNCS:
-            out.append((None, f.id, len(node.args), [k.arg for k in node.keywords if k.arg], node.lineno))
-    return out
+def _reference_calls():
+    with open(os.path.join(FX.HERE, "reference_calls.json")) as f:
+        ref = json.load(f)
+    assert ref["objects"] == list(TARGETS) and ref["functions"] == list(FUNCS)
+    return ref["calls"]
 
 
 def _accepts(fn, n_pos, kws, bound):
@@ -63,10 +52,7 @@ def _accepts(fn, n_pos, kws, bound):
 
 @pytest.mark.parametrize("script", ["inference_t2i.py", "inference_mmu.py", "training/train.py", "training/train_w_clip_vit.py"])
 def test_every_call_of_the_reference_scripts_binds_to_the_drop_in(script):
-    path = os.path.join(REF, script)
-    if not os.path.exists(path):
-        pytest.skip(f"{script} not in this reference tree")
-    calls = _calls(path)
+    calls = _reference_calls()[script]
     assert calls, f"no calls on {list(TARGETS)} found in {script}"
     problems, checked = [], 0
     for obj, meth, n_pos, kws, line in calls:
